@@ -2,8 +2,12 @@
 """bench.py -- the BASELINE.json headline metric: Panda 7-DOF fkine+jacob0 evaluations/s at
 batch 1M (configs[1]: Panda ETS, fp64, seed 0, q ~ U(-pi, pi), 1M rows per GPU).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W]            # this repo's CUDA path
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--dump-outputs DIR]   # this repo's CUDA path
     python bench.py --impl reference [--gpus N] [--steps K] [--warmup W]   # the reference's CPU path
+
+--dump-outputs DIR writes what the last timed step returned (T and J) for a fixed, seeded sample of
+DUMP_ROWS rows as DIR/T.npy and DIR/J.npy (float64, rank 0's shard), so that two builds run with the
+same arguments can be compared output for output.
 
 A "step" is one pass of the hot path over one 1M-row batch: ONE launch of the fused
 fkine+jacob0 kernel (b2k_fkine_jacob0 through the C ABI).  Rows are sharded over ranks with no
@@ -51,6 +55,7 @@ WORKLOAD = "panda_ets_fkine_jacob0_f64_batch1M"
 NVLINK_GBS = 900.0  # nominal NVLink 5 bandwidth per direction per GPU (B200_PROFILING.md)
 PARITY_ROWS = 4096
 IK_PARITY_ROWS = 1024
+DUMP_ROWS = 65536  # --dump-outputs sample: 65536 x (16 + 42) x 8 B = 30 MB
 IK_PROTOCOLS = {  # SURVEY 8d config 4: the notebook protocol and the API default
     "ik_lm_panda_f32_100k_chan0.1": dict(k=0.1, jl=False),
     "ik_lm_panda_f32_100k_chan1.0_jl": dict(k=1.0, jl=True),
@@ -257,6 +262,17 @@ def err_stats(got, ref, atol):
     return float(d.max()), float((d[big] / np.abs(ref[big])).max()) if big.any() else 0.0
 
 
+def dump_outputs(out_dir, dev, **arrays):
+    """Write the same DUMP_ROWS rows (seeded, sorted) of each (ROWS_PER_GPU, ...) device array as out_dir/<name>.npy."""
+    import torch
+
+    os.makedirs(out_dir, exist_ok=True)
+    rows = np.sort(np.random.default_rng(5).choice(ROWS_PER_GPU, DUMP_ROWS, replace=False))
+    idx = torch.from_numpy(rows).to(dev)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a.index_select(0, idx).cpu().numpy())
+
+
 def run_b200(args):
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -347,6 +363,8 @@ def run_b200(args):
     n0 = rtb.launch_count()
     ms_step = time_steps(step, args.steps, W)
     launches = rtb.launch_count() - n0 - W
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, dev, T=T, J=J)  # before the per-step pass below overwrites T and J
     value = ROWS_PER_GPU * world / (ms_step * 1e-3)
     clocks = sampler.summary(windows[-1:])
     per = time_steps(step, min(args.steps, 200), 0, per_step=True)  # distribution, outside `value`
@@ -626,7 +644,10 @@ def main():
     ap.add_argument("--headline-only", action="store_true", help="skip the secondary configs and the gather")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-fused-gather", action="store_true", help="skip the symmetric-memory store-to-root experiment (N>1)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write T and J of the last timed step (a seeded row sample) as DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference(args)
     return run_b200(args)
