@@ -252,9 +252,9 @@ __device__ __forceinline__ void je_col_pri(const Pose<real> &U, real sg, real *c
 //   0 generic: any axis / flip / constant, runtime (uniform) switches.
 //   TRIG = 1 (the IK loop, whose iterates leave [-pi, pi] in some lanes of most warps): fp32 angles are reduced once
 //   and go to the special-function unit whatever their size, so a warp never runs two sincos paths back to back.
-template <typename real, int N, bool WJ, int PROF, int TRIG = 0, typename GetQ>
-__device__ __forceinline__ void chain_forward(const ChainP<real, N> &P, GetQ getq, Pose<real> &T,
-                                              real (*zj)[3], real (*pj)[3])
+// zj / pj are indexed zj[j][i]: register arrays real[N][3], or JRowCols views of a Jacobian row in shared memory.
+template <typename real, int N, bool WJ, int PROF, int TRIG = 0, typename GetQ, typename ZJ, typename PJ>
+__device__ __forceinline__ void chain_forward(const ChainP<real, N> &P, GetQ getq, Pose<real> &T, ZJ zj, PJ pj)
 {
     if constexpr (PROF == 1) {
         real eta[N], sn[N], cs[N];
@@ -340,6 +340,34 @@ __device__ __forceinline__ void jacob0_row(const ChainP<real, N> &P, const Pose<
             row[4 * N + j] = (real)0;
             row[5 * N + j] = (real)0;
         }
+    }
+}
+
+// Rows K0..K0+2 of a row-major 6 x N Jacobian row, column j seen as the 3-vector v[j][0..2] (the indexing of the
+// register stash arrays): lets chain_forward write its stash straight into the Jacobian row in shared memory.
+template <typename real, int N, int K0>
+struct JRowCols {
+    real *row;
+    struct Col {
+        real *p;
+        __device__ __forceinline__ real &operator[](int i) const { return p[i * N]; }
+    };
+    __device__ __forceinline__ Col operator[](int j) const { return Col{row + K0 * N + j}; }
+};
+
+// The DH-like walk's stash written into the row itself (JRowCols<3> for z_j, JRowCols<0> for p_j): rows 3..5 already
+// hold their final values z_j, rows 0..2 hold p_j and are overwritten with z_j x (p_e - p_j) -- the expressions of
+// jacob0_row, so the result is bit-identical to the register form.
+template <typename real, int N>
+__device__ __forceinline__ void jacob0_from_stash(const Pose<real> &T, real *row)
+{
+#pragma unroll
+    for (int j = 0; j < N; j++) {
+        const real z0 = row[3 * N + j], z1 = row[4 * N + j], z2 = row[5 * N + j];
+        const real dx = T.p[0] - row[0 * N + j], dy = T.p[1] - row[1 * N + j], dz = T.p[2] - row[2 * N + j];
+        row[0 * N + j] = fma(z1, dz, -(z2 * dy));
+        row[1 * N + j] = fma(z2, dx, -(z0 * dz));
+        row[2 * N + j] = fma(z0, dy, -(z1 * dx));
     }
 }
 
@@ -562,6 +590,17 @@ __device__ __forceinline__ void prefetch_q_tile_l2(const real *gq, int rows_here
         asm volatile("prefetch.global.L2 [%0];" ::"l"(a));
 }
 
+// Programmatic dependent launch: every fkj kernel is launched with programmatic stream serialization (fkj_launch_pdl),
+// so it may become resident while the previous kernel on the stream is still draining.  griddepcontrol.wait blocks
+// until that kernel has completed and its writes are visible (q may be what it wrote), so it precedes every global
+// access; launch_dependents then lets the next fkj call be scheduled onto the SMs this grid frees.  Both are no-ops
+// when the kernel was launched without the attribute.
+__device__ __forceinline__ void pdl_wait_then_release()
+{
+    asm volatile("griddepcontrol.wait;" ::: "memory");
+    asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
+}
+
 // bytes of per-warp shared memory: [q tile][output stage]
 template <typename real>
 inline size_t fkj_q_bytes(int ldq) { return ((size_t)32 * (ldq | 1) * sizeof(real) + 15) & ~(size_t)15; }
@@ -589,6 +628,7 @@ k_fkj_forward(const __grid_constant__ ChainP<real, N> P, const real *__restrict_
 {
     // dbg (measurement skeletons, b2k_set_variant 2 / 3): bit 0 = skip the chain walk (memory
     // traffic only), bit 1 = skip the output stores (arithmetic only).  0 in normal operation.
+    pdl_wait_then_release();
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int lane = threadIdx.x & 31;
     const int warp = threadIdx.x >> 5;
@@ -720,45 +760,85 @@ __device__ __forceinline__ void backward_walk_dh(const ChainP<real, N> &P, const
 // This kernel is the same walk with everything about the call fixed at compile time: DH-like chain (PROF 1),
 // q rows exactly N wide with jindex j = column j, 16-byte aligned q, one FULL tile per warp.  The launcher uses it
 // for the full tiles of such calls and hands a ragged tail (nrows % 32 rows) to the general kernel.
+//
+// Jacobian stash (SMEM_STASH).  Held in registers, the walk's z_j / p_j stash is 6N reals per lane: 84 of the 128
+// registers of the fp64 Panda kernel, which capped it at 4 resident blocks (16 warps) per SM -- too few to cover a
+// DRAM round trip under the saturated write stream.  So fp64 kernels keep the stash in the lane's own row of the
+// J stage (exactly 6N reals): z_j is written to its final place in rows 3..5 as soon as it is known, p_j to the
+// row 0..2 places as scratch, and jacob0_from_stash finishes the row in place.  The q tile is the front of that stage.
+// The stash's shared accesses run at the row stride of 6N reals.  For odd N the compiler pairs consecutive joints into
+// 16-byte accesses, which are conflict-free at that stride; for even N they would be 2-way (16 B) to 4-way (8 B)
+// bank-conflicted.  So only odd N <= 7 take it (N = 7: 96 registers, 43,008 B per block, 5 blocks per SM), and only in
+// the fused pose + Jacobian kernel: the Jacobian-only one spills 48 B when held to 96 registers.
 template <typename real, int N>
 struct FkjFast {
     static constexpr int QBYTES = 32 * N * (int)sizeof(real);          // multiple of 128
     static constexpr int QUNITS = QBYTES / 16;
+    static constexpr bool SMEM_STASH = sizeof(real) == 8 && (N % 2) == 1 && N <= 7;
     static constexpr int WB_POSE = QBYTES;                                  // per-warp shared memory, pose only
-    static constexpr int WB_JAC = QBYTES + TileStage<real, 6 * N>::BYTES;   // with the Jacobian stage
+    static constexpr int WB_JAC = QBYTES + TileStage<real, 6 * N>::BYTES;   // with the Jacobian stage after the q tile
+    static constexpr int WB_JAC_SS = TileStage<real, 6 * N>::BYTES;         // q tile inside the Jacobian stage
+    __host__ __device__ static constexpr bool stash(bool wt, bool wj) { return wt && wj && SMEM_STASH; }
+    __host__ __device__ static constexpr int wb(bool wt, bool wj) { return !wj ? WB_POSE : (stash(wt, wj) ? WB_JAC_SS : WB_JAC); }
+    __host__ __device__ static constexpr int minb(bool wt, bool wj)
+    {
+        return stash(wt, wj) ? 5 : (wj ? FkjBounds<real, N, true>::MINB : FkjBounds<real, N, false>::MINB);
+    }
 };
 
-template <typename real, int N, bool WT, bool WJ>
-__global__ void __launch_bounds__(B2K_THREADS, FkjBounds<real, N, WJ>::MINB)
-k_fkj_fast(const __grid_constant__ ChainP<real, N> P, const real *__restrict__ q, int ntiles, real *__restrict__ Tout,
-           real *__restrict__ Jout)
+// A lean kernel's q tile: L2 prefetch of the tile `pf_ahead` tiles further on (the launcher passes one resident grid's
+// worth, so that tile's warp starts about one warp lifetime later and finds its q in L2), then 16-byte cp.async of
+// this tile into shared memory.  Returns after the tile has landed and is visible to the whole warp.
+template <typename real, int N>
+__device__ __forceinline__ void lean_load_q(const real *q, int tile, int ntiles, int pf_ahead, real *sq, int lane)
 {
+    typedef FkjFast<real, N> F;
+    if (lane == 0 && tile < ntiles - pf_ahead) {
+        const real *pf = q + (size_t)(tile + pf_ahead) * (32 * N);
+        asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(pf), "r"((unsigned)F::QBYTES) : "memory");
+    }
+    const uint4 *g = reinterpret_cast<const uint4 *>(q + (size_t)tile * (32 * N));
+    uint4 *sdst = reinterpret_cast<uint4 *>(sq);
+#pragma unroll
+    for (int u = 0; u < (F::QUNITS + 31) / 32; u++) {
+        const int idx = u * 32 + lane;
+        if (F::QUNITS % 32 == 0 || idx < F::QUNITS) cp_async16(sdst + idx, g + idx);
+    }
+    cp_async_wait_all();
+    __syncwarp();
+}
+
+template <typename real, int N, bool WT, bool WJ>
+__global__ void __launch_bounds__(B2K_THREADS, FkjFast<real, N>::minb(WT, WJ))
+k_fkj_fast(const __grid_constant__ ChainP<real, N> P, const real *__restrict__ q, int ntiles, int pf_ahead,
+           real *__restrict__ Tout, real *__restrict__ Jout)
+{
+    pdl_wait_then_release();
     extern __shared__ __align__(16) unsigned char smem_raw[];
     typedef FkjFast<real, N> F;
-    constexpr int WB = WJ ? F::WB_JAC : F::WB_POSE;
+    typedef TileStage<real, 6 * N> JS;
+    constexpr bool STASH = F::stash(WT, WJ);
+    static_assert(!STASH || JS::EXACT, "the stash needs the stage to be the exact image of the J block");
     const int lane = threadIdx.x & 31;
     const int warp = threadIdx.x >> 5;
     const int tile = blockIdx.x * B2K_WARPS_PER_BLOCK + warp;
     if (tile >= ntiles) return;
-    unsigned char *wbase = smem_raw + warp * WB;
+    unsigned char *wbase = smem_raw + warp * F::wb(WT, WJ);
     real *sq = reinterpret_cast<real *>(wbase);
-    {
-        const uint4 *g = reinterpret_cast<const uint4 *>(q + (size_t)tile * (32 * N));
-        uint4 *sdst = reinterpret_cast<uint4 *>(sq);
-#pragma unroll
-        for (int u = 0; u < (F::QUNITS + 31) / 32; u++) {
-            const int idx = u * 32 + lane;
-            if (F::QUNITS % 32 == 0 || idx < F::QUNITS) cp_async16(sdst + idx, g + idx);
-        }
-    }
-    cp_async_wait_all();
-    __syncwarp();
+    lean_load_q<real, N>(q, tile, ntiles, pf_ahead, sq, lane);
     real qrow[N];
 #pragma unroll
     for (int j = 0; j < N; j++) qrow[j] = sq[lane * N + j];
+    unsigned char *so = wbase + (STASH ? 0 : F::QBYTES); // the J stage
+    real *srow = reinterpret_cast<real *>(so) + lane * (6 * N); // this lane's row of it (stash form)
     Pose<real> T;
-    real zj[WJ ? N : 1][3], pj[WJ ? N : 1][3];
-    chain_forward<real, N, WJ, 1>(P, [&](int j, int) { return qrow[j]; }, T, zj, pj);
+    if constexpr (STASH) {
+        __syncwarp(); // the q tile is the front of the stage: every lane holds its q row before any lane overwrites it
+        chain_forward<real, N, true, 1>(P, [&](int j, int) { return qrow[j]; }, T, JRowCols<real, N, 3>{srow},
+                                        JRowCols<real, N, 0>{srow});
+    }
+    real zj[WJ && !STASH ? N : 1][3], pj[WJ && !STASH ? N : 1][3];
+    if constexpr (!STASH) chain_forward<real, N, WJ, 1>(P, [&](int j, int) { return qrow[j]; }, T, zj, pj);
     const size_t row = (size_t)tile * 32 + lane;
     if (WT) {
         Pose<real> Tb = T;
@@ -766,11 +846,13 @@ k_fkj_fast(const __grid_constant__ ChainP<real, N> P, const real *__restrict__ q
         store_pose_row<real>(Tb, Tout + row * 16);
     }
     if (WJ) {
-        typedef TileStage<real, 6 * N> JS;
-        unsigned char *so = wbase + F::QBYTES;
-        real jrow[6 * N];
-        jacob0_row<real, N, 1>(P, T, zj, pj, jrow);
-        JS::put_row(so, lane, jrow);
+        if constexpr (STASH) {
+            jacob0_from_stash<real, N>(T, srow);
+        } else {
+            real jrow[6 * N];
+            jacob0_row<real, N, 1>(P, T, zj, pj, jrow);
+            JS::put_row(so, lane, jrow);
+        }
         real *gout = Jout + (size_t)tile * (32 * 6 * N);
         if (!JS::drain_async(so, gout, 32, lane)) {
             __syncwarp();
@@ -784,9 +866,10 @@ k_fkj_fast(const __grid_constant__ ChainP<real, N> P, const real *__restrict__ q
 // lean form of the backward walk (end-effector-frame Jacobian, optional pose): same contract as k_fkj_fast
 template <typename real, int N, bool WT>
 __global__ void __launch_bounds__(B2K_THREADS, FkjBounds<real, N, true>::MINB)
-k_fkj_back_fast(const __grid_constant__ ChainP<real, N> P, const real *__restrict__ q, int ntiles, real *__restrict__ Tout,
-                real *__restrict__ Jout)
+k_fkj_back_fast(const __grid_constant__ ChainP<real, N> P, const real *__restrict__ q, int ntiles, int pf_ahead,
+                real *__restrict__ Tout, real *__restrict__ Jout)
 {
+    pdl_wait_then_release();
     extern __shared__ __align__(16) unsigned char smem_raw[];
     typedef FkjFast<real, N> F;
     const int lane = threadIdx.x & 31;
@@ -795,17 +878,7 @@ k_fkj_back_fast(const __grid_constant__ ChainP<real, N> P, const real *__restric
     if (tile >= ntiles) return;
     unsigned char *wbase = smem_raw + warp * F::WB_JAC;
     real *sq = reinterpret_cast<real *>(wbase);
-    {
-        const uint4 *g = reinterpret_cast<const uint4 *>(q + (size_t)tile * (32 * N));
-        uint4 *sdst = reinterpret_cast<uint4 *>(sq);
-#pragma unroll
-        for (int u = 0; u < (F::QUNITS + 31) / 32; u++) {
-            const int idx = u * 32 + lane;
-            if (F::QUNITS % 32 == 0 || idx < F::QUNITS) cp_async16(sdst + idx, g + idx);
-        }
-    }
-    cp_async_wait_all();
-    __syncwarp();
+    lean_load_q<real, N>(q, tile, ntiles, pf_ahead, sq, lane);
     real eta[N];
 #pragma unroll
     for (int j = 0; j < N; j++) eta[j] = sq[lane * N + j];
@@ -839,6 +912,7 @@ k_fkj_backward(const __grid_constant__ ChainP<real, N> P, const real *__restrict
                float inv_ldq, int qmode, real *__restrict__ Tout, real *__restrict__ Jout, int warp_smem_bytes,
                int q_bytes, int tpw)
 {
+    pdl_wait_then_release();
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int lane = threadIdx.x & 31;
     const int warp = threadIdx.x >> 5;
@@ -932,6 +1006,28 @@ inline int fkj_qmode(const void *q, int ldq)
     return b2k_gcd(ldq, slots) <= 2 ? 1 : 0;
 }
 
+// Launches an fkj kernel with programmatic stream serialization (see pdl_wait_then_release): its blocks may become
+// resident while the previous kernel on the stream drains, which hides the launch gap and the dispatch ramp between
+// consecutive calls.  A runtime that rejects the attribute gets a plain launch.
+template <typename... KArgs, typename... Args>
+inline cudaError_t fkj_launch_pdl(void (*kern)(KArgs...), unsigned grid, size_t smem, cudaStream_t st, Args... args)
+{
+    cudaLaunchAttribute attr[1];
+    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    attr[0].val.programmaticStreamSerializationAllowed = 1;
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3(grid);
+    cfg.blockDim = dim3(B2K_THREADS);
+    cfg.dynamicSmemBytes = smem;
+    cfg.stream = st;
+    cfg.attrs = attr;
+    cfg.numAttrs = 1;
+    if (cudaLaunchKernelEx(&cfg, kern, args...) == cudaSuccess) return cudaSuccess;
+    cudaGetLastError(); // clear the rejection
+    kern<<<grid, B2K_THREADS, smem, st>>>(args...);
+    return cudaGetLastError();
+}
+
 template <typename real, int N>
 int fkj_launch_n(const b2k_chain_s *c, int mode, const real *q, long long nrows, int ldq, const double *base,
                  const double *tool, real *T, real *J, cudaStream_t st)
@@ -972,9 +1068,9 @@ int fkj_launch_n(const b2k_chain_s *c, int mode, const real *q, long long nrows,
         long long grid = (ntiles + B2K_WARPS_PER_BLOCK * tpw - 1) / (B2K_WARPS_PER_BLOCK * tpw);
         if (grid < 1) grid = 1;
         if (grid > 0x7fffffffLL || tpw > 0x7fffffffLL) { b2k_set_error("fkj: batch too large for one launch"); return B2K_ERR_INVALID; }
-        kern<<<(unsigned)grid, B2K_THREADS, smem, st>>>(P, q, nrows, ldq, inv_ldq, qmode, T, J, (int)wsm, (int)qb, (int)tpw, extra...);
+        B2K_CUDA(fkj_launch_pdl(kern, (unsigned)grid, smem, st, P, q, nrows, ldq, inv_ldq, qmode, T, J, (int)wsm, (int)qb,
+                                (int)tpw, extra...));
         b2k_count_launch();
-        B2K_CUDA(cudaGetLastError());
         return B2K_OK;
     };
     auto launch = [&](auto kern) -> int { return launch_impl(kern, dbg); };   // forward kernels take dbg
@@ -988,16 +1084,16 @@ int fkj_launch_n(const b2k_chain_s *c, int mode, const real *q, long long nrows,
             int per_sm = b2k_blocks_per_sm((const void *)kern, B2K_THREADS, fsmem);
             if (per_sm < 1) return per_sm < 0 ? per_sm : (b2k_set_error("fkj fast kernel does not fit on an SM (smem %zu B)", fsmem), B2K_ERR_INVALID);
             const unsigned grid = (unsigned)((nfull + B2K_WARPS_PER_BLOCK - 1) / B2K_WARPS_PER_BLOCK);
-            kern<<<grid, B2K_THREADS, fsmem, st>>>(P, q, nfull, T, J);
+            const int pf_ahead = b2k_num_sms() * per_sm * B2K_WARPS_PER_BLOCK; // one resident grid of tiles (lean_load_q)
+            B2K_CUDA(fkj_launch_pdl(kern, grid, fsmem, st, P, q, nfull, pf_ahead, T, J));
             b2k_count_launch();
-            B2K_CUDA(cudaGetLastError());
             return B2K_OK;
         };
         typedef FkjFast<real, N> F;
         int rc;
         if (wje) rc = wt ? launch_fast(k_fkj_back_fast<real, N, true>, (size_t)F::WB_JAC * B2K_WARPS_PER_BLOCK)
                          : launch_fast(k_fkj_back_fast<real, N, false>, (size_t)F::WB_JAC * B2K_WARPS_PER_BLOCK);
-        else if (wt && wj0) rc = launch_fast(k_fkj_fast<real, N, true, true>, (size_t)F::WB_JAC * B2K_WARPS_PER_BLOCK);
+        else if (wt && wj0) rc = launch_fast(k_fkj_fast<real, N, true, true>, (size_t)F::wb(true, true) * B2K_WARPS_PER_BLOCK);
         else if (wt) rc = launch_fast(k_fkj_fast<real, N, true, false>, (size_t)F::WB_POSE * B2K_WARPS_PER_BLOCK);
         else rc = launch_fast(k_fkj_fast<real, N, false, true>, (size_t)F::WB_JAC * B2K_WARPS_PER_BLOCK);
         const long long done = (long long)nfull * 32;
