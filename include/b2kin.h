@@ -103,6 +103,11 @@ int b2k_chain_info(b2k_chain_t chain, int *n, int *m, int *q_width);
  * Replaces fknm.ETS_fkine (fknm.cpp:923-1064 -> _ETS_fkine methods.cpp:318-352):
  *   T[i] = base * prod_k ET_k(q[i, jindex_k]) * tool
  * ldq = row stride of q in elements (>= q_width).
+ * Output alignment, here and in b2k_jacob0 / b2k_jacobe / b2k_fkine_jacob0 / b2k_fkine_jacobe (a misaligned
+ * output is refused with B2K_ERR_INVALID; every cudaMalloc / torch allocation qualifies):
+ *   T (N,4,4): 32-byte aligned;
+ *   J (N,6,n): 16-byte aligned for B2K_F64 and for B2K_F32 with even n, 8-byte aligned for B2K_F32 with odd n.
+ * q needs only the alignment of its element type.
  */
 int b2k_fkine(b2k_chain_t chain, int dtype, const void *q, int64_t N, int64_t ldq,
               const double *base, const double *tool, void *T, void *stream);
@@ -121,21 +126,22 @@ int b2k_fkine_frames(b2k_chain_t chain, int dtype, const void *q, int64_t N, int
 
 /* Replaces fknm.ETS_jacob0 (fknm.cpp:785-850 -> _ETS_jacob0 methods.cpp:112-216), batched:
  * J[i] = geometric Jacobian in the chain's start frame, (6,n) row-major per row; no base
- * (reference RobotKinematics.py:158), tool included. */
+ * (reference RobotKinematics.py:158), tool included.  J aligned as for b2k_fkine above. */
 int b2k_jacob0(b2k_chain_t chain, int dtype, const void *q, int64_t N, int64_t ldq,
                const double *tool, void *J, void *stream);
 
 /* Replaces fknm.ETS_jacobe (fknm.cpp:852-921 -> _ETS_jacobe methods.cpp:219-316), batched:
- * Jacobian in the end-effector frame. */
+ * Jacobian in the end-effector frame.  J aligned as for b2k_fkine above. */
 int b2k_jacobe(b2k_chain_t chain, int dtype, const void *q, int64_t N, int64_t ldq,
                const double *tool, void *J, void *stream);
 
 /* Fused pose + base-frame Jacobian in one pass over q (the BASELINE headline op):
- * T as b2k_fkine (base and tool applied), J as b2k_jacob0 (tool applied, no base). */
+ * T as b2k_fkine (base and tool applied), J as b2k_jacob0 (tool applied, no base).  T 32-byte aligned, J as for
+ * b2k_fkine above. */
 int b2k_fkine_jacob0(b2k_chain_t chain, int dtype, const void *q, int64_t N, int64_t ldq,
                      const double *base, const double *tool, void *T, void *J, void *stream);
 
-/* Fused pose + end-effector-frame Jacobian. */
+/* Fused pose + end-effector-frame Jacobian.  T 32-byte aligned, J as for b2k_fkine above. */
 int b2k_fkine_jacobe(b2k_chain_t chain, int dtype, const void *q, int64_t N, int64_t ldq,
                      const double *base, const double *tool, void *T, void *J, void *stream);
 

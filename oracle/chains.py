@@ -267,6 +267,53 @@ def pack_rne(links, mdh=False):
     return L
 
 
+def random_se3(rng, reach=0.5):
+    """A general rigid transform: rotations about all three axes and a translation in [-reach, reach]^3."""
+    return (trotz(rng.uniform(-math.pi, math.pi)) @ troty(rng.uniform(-math.pi, math.pi))
+            @ trotx(rng.uniform(-math.pi, math.pi)) @ transl(*rng.uniform(-reach, reach, 3)))
+
+
+DH_ALPHAS = (0.0, math.pi / 2, -math.pi / 2, None)  # None: alpha drawn from U(-pi, pi)
+
+
+def dh_like_chain(rng, n, tail=True):
+    """A random chain of the shape the kernels treat as DH-like: a general SE(3) head A_0, n unflipped Rz joints,
+    inter-joint constants transl(x, y, z) @ trotx(alpha) and, with `tail`, a general SE(3) tail.  Without it nothing
+    follows the last joint.  The alphas cycle from a random start through 0 (a pure translation), +-pi/2 (cos(alpha)
+    stays 6.1e-17, not 0) and a random angle, so every kind appears once a chain has four inter-joint constants."""
+    b = Builder()
+    b.se3(random_se3(rng))
+    k0 = int(rng.integers(0, len(DH_ALPHAS)))
+    for j in range(n):
+        if j > 0:
+            alpha = DH_ALPHAS[(k0 + j) % len(DH_ALPHAS)]
+            if alpha is None:
+                alpha = float(rng.uniform(-math.pi, math.pi))
+            b.se3(transl(*rng.uniform(-0.5, 0.5, 3)) @ trotx(alpha))
+        b.joint(RZ)
+    if tail:
+        b.se3(random_se3(rng))
+    return b.desc()
+
+
+def perturb_joint(desc, k, flip=None, axis=None):
+    """A copy of a chain description with the k-th joint flipped and/or moved to another axis."""
+    d = {key: (v.copy() if isinstance(v, np.ndarray) else v) for key, v in desc.items()}
+    i = int(np.flatnonzero(d["isjoint"])[k])
+    if flip is not None:
+        d["flip"][i] = int(flip)
+    if axis is not None:
+        d["axis"][i] = int(axis)
+    return d
+
+
+def chain_reach(desc, *extra):
+    """Sum of the translation lengths of a chain's constants and of any extra 4x4 transforms (base, tool): a bound on
+    how far the end effector can be from the origin, the scale of the absolute errors of poses and Jacobians."""
+    Ts = [T for T, j in zip(desc["T"], desc["isjoint"]) if not j] + [T for T in extra if T is not None]
+    return float(sum(np.linalg.norm(np.asarray(T)[:3, 3]) for T in Ts))
+
+
 def random_chain(rng, n_joints=6, with_flips=True, extra_consts=True):
     """A random serial chain exercising all six ET kinds, flips, constant runs and SE3 constants."""
     b = Builder()
